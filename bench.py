@@ -2,7 +2,7 @@
 """bench.py - self-play throughput (BASELINE.json metric: env-steps/s and MCTS simulations/s) on N B200s.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl ours|reference]
-                  [--extras a,b,c | --no-extras] [--no-cpu-baseline] [--no-loop]
+                  [--extras a,b,c | --no-extras] [--no-cpu-baseline] [--no-loop] [--dump-outputs DIR]
 
 What is timed
 -------------
@@ -15,6 +15,11 @@ search would otherwise give a 12 ms sample); the L2 is flushed (256 MiB write, u
 `loop`  = env-steps/s of the WHOLE self-play loop through the public `SelfPlay` API (SURVEY.md 8d's full definition:
           search + environment step + action sampling + GameHistory hand-over), timed >= 1 s;
 `workloads` = the same sub-lines for the other BASELINE configs at this --gpus N.
+
+--dump-outputs DIR writes what the last timed search of the headline workload returned (visit counts, root values,
+root priors, ...; the search's SearchOutput arrays) as DIR/<name>.npy.  Inputs, weights and the search seed are fixed,
+and the last timed search always runs on the same one of the rotating input batches, so two runs with the same
+arguments, or two builds of the project, can be compared output for output.
 
 N=1 headline workload: BASELINE.json configs[1] - CartPole, fully-connected net, num_simulations=50, 4096 parallel
 games per GPU (weak scaling: every rank owns its own games; no data-path collective - one all-gather of per-rank
@@ -317,8 +322,8 @@ def run_workload(name, args, D, rank, local_rank, world, with_loop, headline):
         est = D.max([est])[0]
         inner = max(1, int(math.ceil(MIN_TIMED_SECONDS / max(est * steps, 1e-9))))
         D.barrier()
-        per_search, per_step, kern, visits = [], [], 0.0, None
-        i = 0
+        per_search, per_step, kern, out = [], [], 0.0, None
+        i = -(steps * inner) % n_batches          # the last timed search runs on the last batch, whatever `inner` is
         for _ in range(steps):
             acc = 0.0
             for _ in range(inner):
@@ -327,11 +332,10 @@ def run_workload(name, args, D, rank, local_rank, world, with_loop, headline):
                 acc += dt
                 per_search.append(1000.0 * dt)
                 kern += out.device_ms
-                visits = out.visit_counts
             per_step.append(1000.0 * acc)
         D.barrier()
         return dict(wall=sum(per_step) / 1000.0, kern_ms=kern, searches=steps * inner, inner=inner,
-                    per_search=per_search, per_step=per_step, visits=visits)
+                    per_search=per_search, per_step=per_step, last=out)
 
     clocks = ClockSampler(local_rank) if headline else None
     if clocks:
@@ -343,8 +347,10 @@ def run_workload(name, args, D, rank, local_rank, world, with_loop, headline):
     launches = eng.launch_count - launches0
     graph_parts = eng.graph_partitions
     clk = clocks.stop() if clocks else None
+    if headline and rank == 0 and args.dump_outputs:
+        dump_outputs(dv["last"], args.dump_outputs)
     hv = timed(search_host, args.steps, args.warmup)
-    assert int(numpy.asarray(hv["visits"]).sum()) == B * N
+    assert int(numpy.asarray(hv["last"].visit_counts).sum()) == B * N
     kernel_split = {}
     if game != "cartpole":
         eng.kernel_timing(True)
@@ -438,6 +444,25 @@ def run_workload(name, args, D, rank, local_rank, world, with_loop, headline):
     return sub
 
 
+DUMP_FIELDS = ("visit_counts", "root_value", "root_predicted_value", "max_tree_depth", "tie_count", "root_priors",
+               "value_range")
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out, directory):
+    """Writes the SearchOutput arrays of one search as DIR/<field>.npy (integers as float64, which holds them exactly),
+    so that two builds can be compared output for output on the same seeded inputs."""
+    arrays = {}
+    for f in DUMP_FIELDS:
+        a = getattr(out, f)
+        a = a.cpu().numpy() if hasattr(a, "cpu") else numpy.asarray(a)
+        arrays[f] = a if a.dtype in (numpy.float32, numpy.float64) else a.astype(numpy.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= DUMP_MAX_BYTES
+    os.makedirs(directory, exist_ok=True)
+    for f, a in arrays.items():
+        numpy.save(os.path.join(directory, f + ".npy"), a)
+
+
 def saturation_curve(cfg, spec, N, device, dev):
     """Search throughput of the fused FC kernel at larger batches than the BASELINE's 4096 games: the headline launch
     lasts one game's chain of N dependent simulations with 28 games per SM in flight; more games per SM fill the issue
@@ -514,6 +539,8 @@ def main():
     ap.add_argument("--no-saturation", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the headline workload's last timed search outputs (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "ours":
         args.warmup = max(args.warmup, 3)

@@ -596,8 +596,75 @@ def main_round2():
     print("network fixtures (batch 64, stress weights) written")
 
 
+def priority_key(name, td, discount, alpha, reanalysed):
+    return f"{name}/td{td}/discount{discount}/alpha{alpha}/reanalysed{int(reanalysed)}"
+
+
+# (game, td_steps, discount, PER_alpha, reanalysed values): one- and two-player games, short and long td horizons
+PRIORITY_CASES = [("tictactoe", 20, 1, 0.5, False), ("cartpole", 50, 0.997, 0.5, False),
+                  ("cartpole", 7, 0.9, 1.0, True), ("connect4", 3, 1, 0.7, True)]
+PRIORITY_LENGTHS = (1, 2, 9, 42, 130)
+
+
+def main_replay():
+    """replay_buffer.json: what the reference's ReplayBuffer computes from game histories.
+
+    * ``priorities``: ``save_game``'s PER priorities and game priority of random histories
+      (``tests/helpers.random_history``, RandomState(4), game lengths PRIORITY_LENGTHS per case).
+    * ``batch``: ``save_game`` + ``get_batch`` (batch_size 8) over six TicTacToe games played by THIS package's
+      ``SelfPlay`` (seed 1, 4 parallel games, 8 simulations, synthetic weights seed 0, the oracle-backed test double
+      in place of the GPU engine), each passed through pickle first."""
+    import copy
+    import pickle
+    sys.path.insert(0, os.path.join(ROOT, "tests"))
+    from fake_engine import FakeSearchEngine
+    from helpers import random_history
+    from muzero_general_b200 import self_play as mysp
+    import muzero_general_b200.games as mygames
+    _, _, ref_rb, _ = load_reference()
+    ck = {"num_played_games": 0, "num_played_steps": 0}
+
+    priorities = {}
+    for name, td, discount, alpha, reanalysed in PRIORITY_CASES:
+        cfg = load_reference_game(name).MuZeroConfig()
+        cfg.td_steps, cfg.discount, cfg.PER_alpha, cfg.PER = td, discount, alpha, True
+        rs = numpy.random.RandomState(4)
+        rows = []
+        for T in PRIORITY_LENGTHS:
+            gh = random_history(rs, cfg, T, len(cfg.players))
+            if reanalysed:
+                gh.reanalysed_predicted_root_values = rs.standard_normal(T).astype(numpy.float32)
+            ref_rb.ReplayBuffer(copy.deepcopy(ck), {}, cfg).save_game(gh)
+            assert gh.priorities.dtype == numpy.float32
+            rows.append(dict(T=T, priorities=f64list(gh.priorities), game_priority=float(gh.game_priority)))
+        priorities[priority_key(name, td, discount, alpha, reanalysed)] = rows
+
+    mod = mygames.load_game_module("tictactoe")
+    my_cfg = mod.MuZeroConfig()
+    my_cfg.num_parallel_games, my_cfg.num_simulations = 4, 8
+    mysp.SearchEngine = FakeSearchEngine
+    worker = mysp.SelfPlay({"weights": synthetic_weights(netspec_from_config(my_cfg), 0)}, mod.Game, my_cfg, 1)
+    games = worker.play_games(6, 1.0)
+    cfg = load_reference_game("tictactoe").MuZeroConfig()
+    cfg.num_simulations, cfg.batch_size, cfg.train_on_gpu = 8, 8, False
+    buf = ref_rb.ReplayBuffer(dict(ck, weights=None), {}, cfg)
+    for gh in games:
+        buf.save_game(pickle.loads(pickle.dumps(gh)))
+    index_batch, (obs_b, act_b, val_b, rew_b, pol_b, _, _) = buf.get_batch()
+    batch = dict(num_games=len(games), index=[[int(g), int(p)] for g, p in index_batch],
+                 priorities=[f64list(buf.buffer[g].priorities) for g in range(len(games))],
+                 game_priority=[float(buf.buffer[g].game_priority) for g in range(len(games))],
+                 observation=[numpy.asarray(o, dtype=numpy.float64).ravel().tolist() for o in obs_b],
+                 action=[[int(a) for a in r] for r in act_b], value=[f64list(r) for r in val_b],
+                 reward=[f64list(r) for r in rew_b], policy=[[f64list(p) for p in r] for r in pol_b])
+    json.dump(dict(priorities=priorities, batch=batch), open(os.path.join(OUT, "replay_buffer.json"), "w"))
+    print("replay buffer fixtures written")
+
+
 if __name__ == "__main__":
     if "--round2" in sys.argv:
         main_round2()
+    elif "--replay" in sys.argv:
+        main_replay()
     else:
         main()

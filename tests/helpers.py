@@ -1,4 +1,5 @@
-"""Shared test helpers: teacher tables from golden traces, oracle replays."""
+"""Shared test helpers (also used by oracle/gen_golden.py): teacher tables from golden traces, oracle replays,
+random game histories."""
 import numpy
 
 from oracle import mcts as om
@@ -46,6 +47,20 @@ def oracle_replay(params, legal, to_play, root, sims, noise, first_index, seed=0
         tie_fn=lambda n_tied, ctx: philox.tie_index(seed, game, move, ctx[0], ctx[1], n_tied))
     res = om.TreeSearch(params).run(ev, None, legal, to_play, noise is not None, draws)
     return res, draws
+
+
+def random_history(rs, cfg, T, players):
+    """A GameHistory of T random moves (random observations, rewards, visit distributions and root values)."""
+    from muzero_general_b200 import self_play as sp
+    gh = sp.GameHistory()
+    A = len(cfg.action_space)
+    gh.action_history = [0] + [int(a) for a in rs.randint(0, A, T)]
+    gh.observation_history = [rs.random_sample(cfg.observation_shape).astype(numpy.float32) for _ in range(T + 1)]
+    gh.reward_history = [0] + [float(r) for r in rs.choice([0.0, 1.0, -1.0, 0.5], T)]
+    gh.to_play_history = [int(i % players) for i in range(T + 1)] if players > 1 else [0] * (T + 1)
+    cv = rs.random_sample((T, A)); gh.child_visits = (cv / cv.sum(1, keepdims=True)).tolist()
+    gh.root_values = [float(v) for v in rs.standard_normal(T)]
+    return gh
 
 
 def random_teacher(rs, n, N, A, reward_scale=1.0, legal=None):

@@ -1,62 +1,55 @@
 """Bulk callers either side of the self-play path (muzero_general_b200/reanalyse.py) on the CPU: PER priorities against
-the unmodified reference ReplayBuffer, batched Reanalyse against the oracle network."""
+those the unmodified reference ReplayBuffer computed (recorded golden data), batched Reanalyse against the oracle network."""
 import copy
 
 import numpy
 import pytest
 import torch
 
-from conftest import weights_for
+from conftest import golden_json, weights_for
 from fake_engine import FakeSearchEngine
+from helpers import random_history
 from muzero_general_b200 import reanalyse as ra
-from muzero_general_b200 import self_play as sp
 from muzero_general_b200.games import load_game_module
 from muzero_general_b200.netspec import netspec_from_config
-from oracle.refload import reference_available
+from oracle.gen_golden import PRIORITY_CASES, PRIORITY_LENGTHS, priority_key
 
 torch.set_num_threads(1)
 
 
-def _random_history(rs, cfg, T, players):
-    gh = sp.GameHistory()
-    A = len(cfg.action_space)
-    gh.action_history = [0] + [int(a) for a in rs.randint(0, A, T)]
-    gh.observation_history = [rs.random_sample(cfg.observation_shape).astype(numpy.float32) for _ in range(T + 1)]
-    gh.reward_history = [0] + [float(r) for r in rs.choice([0.0, 1.0, -1.0, 0.5], T)]
-    gh.to_play_history = [int(i % players) for i in range(T + 1)] if players > 1 else [0] * (T + 1)
-    cv = rs.random_sample((T, A)); gh.child_visits = (cv / cv.sum(1, keepdims=True)).tolist()
-    gh.root_values = [float(v) for v in rs.standard_normal(T)]
-    return gh
+class _RecordingBuffer:
+    def __init__(self):
+        self.saved = []
+
+    def save_game(self, game_history, shared_storage=None):
+        self.saved.append(game_history)
 
 
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference (not present on the GPU box)")
-@pytest.mark.parametrize("name,td,discount,alpha,reanalysed", [("tictactoe", 20, 1, 0.5, False), ("cartpole", 50, 0.997, 0.5, False),
-                                                               ("cartpole", 7, 0.9, 1.0, True), ("connect4", 3, 1, 0.7, True)])
+@pytest.mark.parametrize("name,td,discount,alpha,reanalysed", PRIORITY_CASES)
 def test_bulk_priorities_equal_the_reference_save_game(name, td, discount, alpha, reanalysed):
     """initial_priorities == what the unmodified ReplayBuffer.save_game computes, bit for bit (float32 priorities, game
-    priority), for one- and two-player games, with and without reanalysed values, short and long td horizons."""
-    from oracle.refload import load_reference, load_reference_game
-    _, _, ref_rb, _ = load_reference()
-    ref_cfg = load_reference_game(name).MuZeroConfig()
-    ref_cfg.td_steps, ref_cfg.discount, ref_cfg.PER_alpha, ref_cfg.PER = td, discount, alpha, True
-    ck = {"num_played_games": 0, "num_played_steps": 0}
+    priority; recorded in tests/golden/replay_buffer.json by oracle/gen_golden.py --replay), for one- and two-player
+    games, with and without reanalysed values, short and long td horizons."""
+    want = golden_json("replay_buffer.json")["priorities"][priority_key(name, td, discount, alpha, reanalysed)]
+    cfg = load_game_module(name).MuZeroConfig()
+    cfg.td_steps, cfg.discount, cfg.PER_alpha, cfg.PER = td, discount, alpha, True
     rs = numpy.random.RandomState(4)
-    for T in (1, 2, 9, 42, 130):
-        gh = _random_history(rs, ref_cfg, T, len(ref_cfg.players))
+    assert [w["T"] for w in want] == list(PRIORITY_LENGTHS)
+    for T, w in zip(PRIORITY_LENGTHS, want):
+        gh = random_history(rs, cfg, T, len(cfg.players))
         if reanalysed:
             gh.reanalysed_predicted_root_values = rs.standard_normal(T).astype(numpy.float32)
-        mine, top = ra.initial_priorities(copy.deepcopy(gh), ref_cfg)
-        buf = ref_rb.ReplayBuffer(copy.deepcopy(ck), {}, ref_cfg)
-        theirs = copy.deepcopy(gh)
-        buf.save_game(theirs)
-        assert mine.dtype == theirs.priorities.dtype == numpy.float32
-        assert numpy.array_equal(mine, theirs.priorities), (name, T)
-        assert top == theirs.game_priority
-        # and save_games attaches them so that the reference keeps them as they are
-        buf2 = ref_rb.ReplayBuffer(copy.deepcopy(ck), {}, ref_cfg)
-        g2 = copy.deepcopy(gh)
-        ra.save_games(buf2, [g2], ref_cfg)
-        assert numpy.array_equal(buf2.buffer[0].priorities, theirs.priorities) and buf2.num_played_steps == T
+        theirs = numpy.array(w["priorities"], dtype=numpy.float32)
+        assert numpy.array_equal(theirs, w["priorities"])               # the fixture holds float32 values exactly
+        mine, top = ra.initial_priorities(copy.deepcopy(gh), cfg)
+        assert mine.dtype == numpy.float32
+        assert numpy.array_equal(mine, theirs), (name, T)
+        assert top == w["game_priority"]
+        # and save_games attaches them before the buffer's save_game sees the game (which then keeps them as they are)
+        buf = _RecordingBuffer()
+        ra.save_games(buf, [copy.deepcopy(gh)], cfg)
+        assert len(buf.saved) == 1 and numpy.array_equal(buf.saved[0].priorities, theirs)
+        assert buf.saved[0].game_priority == w["game_priority"]
 
 
 def test_batched_reanalyse_matches_per_game_inference(monkeypatch):
@@ -70,7 +63,7 @@ def test_batched_reanalyse_matches_per_game_inference(monkeypatch):
     spec = netspec_from_config(cfg)
     w = weights_for("tictactoe", spec)
     rs = numpy.random.RandomState(2)
-    games = [_random_history(rs, cfg, T, 2) for T in (1, 5, 9, 3)]
+    games = [random_history(rs, cfg, T, 2) for T in (1, 5, 9, 3)]
     for g in games:
         g.observation_history = [rs.randint(0, 2, cfg.observation_shape).astype(numpy.int32) for _ in g.observation_history]
     actor = ra.Reanalyse({"weights": w, "num_reanalysed_games": 0}, cfg, max_positions=7)      # forces several chunks

@@ -1,7 +1,6 @@
 """Host-side self-play logic on the CPU (search supplied by the oracle-backed test double):
-draw order, GameHistory format, batched lockstep play, consumption by the reference's own
-ReplayBuffer / Trainer when the reference is present."""
-import copy
+draw order, GameHistory format, batched lockstep play, the training batch the reference's own
+ReplayBuffer builds from our histories (recorded golden data)."""
 import pickle
 
 import numpy
@@ -13,7 +12,6 @@ from fake_engine import FakeSearchEngine
 from muzero_general_b200 import self_play as sp
 from muzero_general_b200.games import load_game_module
 from muzero_general_b200.netspec import netspec_from_config
-from oracle.refload import reference_available
 
 torch.set_num_threads(1)
 
@@ -113,36 +111,34 @@ def test_fast_rng_mode_and_max_moves(fake_engine):
         assert g.observation_history[0].shape == (1, 1, 4) and g.reward_history[1] == 1.0
 
 
-@pytest.mark.skipif(not reference_available(), reason="needs /root/reference (not present on the GPU box)")
-def test_reference_replay_buffer_and_trainer_consume_our_histories(fake_engine):
-    """The unmodified reference ReplayBuffer.save_game/get_batch and Trainer.update_weights accept
-    GameHistory objects produced by this package (SURVEY.md 8c 'consumer acceptance')."""
-    from oracle.refload import load_reference, load_reference_game
-    ref_sp, ref_models, ref_rb, ref_trainer = load_reference()
-    ref_cfg = load_reference_game("tictactoe").MuZeroConfig()
-    ref_cfg.num_simulations = 8
-    ref_cfg.batch_size = 8
-    ref_cfg.train_on_gpu = False
+def test_our_histories_give_the_reference_replay_buffer_batch(fake_engine):
+    """GameHistory objects produced by this package, passed through pickle (the Ray boundary), yield the training
+    batch the unmodified reference ReplayBuffer.save_game / get_batch built from the same games (SURVEY.md 8c
+    'consumer acceptance'; recorded in tests/golden/replay_buffer.json by oracle/gen_golden.py --replay): the
+    priorities it attached, and at every sampled position the stacked observation and, for each unroll step inside
+    the game, the target value, reward, policy and action."""
+    from muzero_general_b200 import reanalyse as ra
+    want = golden_json("replay_buffer.json")["batch"]
     worker, cfg = _worker("tictactoe", 1, num_parallel_games=4, num_simulations=8)
-    games = worker.play_games(6, 1.0)
-    spec = netspec_from_config(cfg)
-    ck = {"weights": {k: torch.from_numpy(numpy.asarray(v)) for k, v in weights_for("tictactoe", spec).items()},
-          "optimizer_state": None, "training_step": 0, "num_played_games": 0, "num_played_steps": 0,
-          "num_reanalysed_games": 0}
-    buf = ref_rb.ReplayBuffer(copy.deepcopy(ck), {}, ref_cfg)
-    for gh in games:
-        gh = pickle.loads(pickle.dumps(gh))                # survives the Ray/pickle boundary
-        buf.save_game(gh)
-        assert gh.priorities is not None and gh.game_priority is not None
-    assert buf.num_played_games == len(games)
-    index_batch, batch = buf.get_batch()
-    obs_b, act_b, val_b, rew_b, pol_b, w_b, grad_b = batch
-    K = ref_cfg.num_unroll_steps + 1
-    assert numpy.asarray(obs_b).shape == (8, 3, 3, 3) and numpy.asarray(act_b).shape == (8, K)
-    assert numpy.asarray(pol_b).shape == (8, K, 9) and numpy.asarray(val_b).shape == (8, K)
-    tr = ref_trainer.Trainer(copy.deepcopy(ck), ref_cfg)
-    priorities, total_loss, value_loss, reward_loss, policy_loss = tr.update_weights(batch)
-    assert numpy.isfinite(total_loss)
+    games = [pickle.loads(pickle.dumps(gh)) for gh in worker.play_games(6, 1.0)]
+    assert len(games) == want["num_games"]
+    for gh, pri, top in zip(games, want["priorities"], want["game_priority"]):
+        mine, mine_top = ra.initial_priorities(gh, cfg)
+        assert numpy.array_equal(mine, numpy.array(pri, numpy.float32)) and mine_top == top
+    assert len(want["index"]) == 8
+    for row, (g, pos) in enumerate(want["index"]):
+        gh = games[g]
+        obs = gh.get_stacked_observations(pos, cfg.stacked_observations, len(cfg.action_space))
+        assert numpy.asarray(obs, dtype=numpy.float64).ravel().tolist() == want["observation"][row]
+        values = ra.target_values(gh, cfg)
+        for k in range(cfg.num_unroll_steps + 1):
+            i = pos + k
+            if i >= len(gh.root_values):
+                break
+            assert float(values[i]) == want["value"][row][k], (row, k)
+            assert float(gh.reward_history[i]) == want["reward"][row][k]
+            assert [float(p) for p in gh.child_visits[i]] == want["policy"][row][k]
+            assert int(gh.action_history[i]) == want["action"][row][k]
 
 
 class _Storage:
