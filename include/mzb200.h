@@ -306,7 +306,10 @@ typedef struct MzSelfPlayPeek {
  *   int64 game_id; int32 slot; int32 length T; int32 first_to_play; int32 obs_elems O; int32 actions A; int32 bytes;
  *   double root_value[T]; int32 visit_counts[T][A]; int32 action[T]; float reward[T]; int32 to_play[T] (after the move);
  *   float priority[T] (zeros unless td_steps > 0); float observation[T+1][O] (index 0 = reset observation); padding to 8.
- * = the fields of GameHistory (self_play.py:479-511) minus the dummy first entries. */
+ * = the fields of GameHistory (self_play.py:479-511) minus the dummy first entries.
+ * A move of the hard-coded opponent (mz_selfplay_set_opponent) is recorded like any other move, with root_value NaN and
+ * all visit counts 0 (a searched move always sums to num_simulations): the reference stores no search statistics for it
+ * (store_search_statistics(None, ...), self_play.py:175,496-511). */
 #define MZ_STAGED_HEADER_BYTES 32
 
 /* replaces the per-move body of SelfPlay.play_game / continuous_self_play for a whole batch (self_play.py:31-183) */
@@ -321,6 +324,23 @@ int mz_selfplay_wait(MzHandle* h, MzSelfPlayStats* stats);
  * {byte offset of the game's block, (slot << 32) | length}, so a consumer can address any game without walking. */
 int mz_selfplay_drain(MzHandle* h, const void** data, uint64_t* bytes, int32_t* n_games, const uint64_t** index);
 int mz_selfplay_peek(MzHandle* h, const MzSelfPlayPeek* out);
+
+/* Evaluation games (self_play.py:54-90, muzero.py:369-424): MuZero plays the side muzero_player, a hard-coded opponent the
+ * other one.  MZ_OPPONENT_EXPERT = the reference's expert scan (games/tictactoe.py:310-349, games/connect4.py:307-348): a
+ * move that completes a line of the side to move, else one that blocks the other side, else a uniformly random legal
+ * move; MZ_OPPONENT_RANDOM = a uniformly random legal move.  The random move is floor(u * n_legal) over the legal
+ * actions in ascending order with u a Philox uniform keyed (seed, game id, move) - numpy.random.choice's distribution,
+ * not its stream.  Only MuZero's moves are searched: the opponent replies in the same move, so every search sees
+ * MuZero to move; env_steps counts the moves of both sides.  Board games only (not CartPole), td_steps == 0,
+ * max_moves >= 2.  MZ_OPPONENT_SELF (the default) is ordinary self-play. */
+enum { MZ_OPPONENT_SELF = 0, MZ_OPPONENT_EXPERT = 1, MZ_OPPONENT_RANDOM = 2 };
+/* after mz_selfplay_begin, before the first move; plays the opponent's opening move where it moves first */
+int mz_selfplay_set_opponent(MzHandle* h, int32_t opponent, int32_t muzero_player);
+/* the device expert / random policy on n given positions (board [n][H*W] int8 with values +1/-1/0, row 0 = the bottom
+ * row, player [n] = +1/-1, uniform [n] = the default-move draw); one warp per position, same device function as the step
+ * kernel.  action [n] receives the move (-1 for a position without a legal action). */
+int mz_debug_opponent_action(int device, int32_t env, int32_t opponent, int32_t n, const int8_t* board,
+                             const int8_t* player, const double* uniform, int32_t* action);
 
 #ifdef __cplusplus
 }

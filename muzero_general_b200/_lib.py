@@ -13,7 +13,7 @@ MZ_MAX_LAYERS = 8
 MZ_MAX_ACTIONS = 128
 MZ_MEM_HOST, MZ_MEM_DEVICE = 0, 1
 MZ_FLAG_KEEP_TREE, MZ_FLAG_STEPWISE, MZ_FLAG_CONTINUE = 1, 2, 4
-MZ_EUNSUPPORTED = -3
+MZ_EINVAL, MZ_EUNSUPPORTED, MZ_ESTATE = -1, -3, -4
 
 _L = C.c_int32 * MZ_MAX_LAYERS
 
@@ -109,6 +109,7 @@ class MzSelfPlayPeek(C.Structure):
 
 
 MZ_ENV_CARTPOLE, MZ_ENV_TICTACTOE, MZ_ENV_CONNECT4 = 0, 1, 2
+MZ_OPPONENT_SELF, MZ_OPPONENT_EXPERT, MZ_OPPONENT_RANDOM = 0, 1, 2
 MZ_STAGED_HEADER_BYTES = 32
 
 # every symbol include/mzb200.h declares: (name, restype, argtypes)
@@ -138,6 +139,9 @@ SYMBOLS = [
     ("mz_selfplay_drain", C.c_int, [C.c_void_p, C.POINTER(C.c_void_p), C.POINTER(C.c_uint64), C.POINTER(C.c_int32),
                                     C.POINTER(C.c_void_p)]),
     ("mz_selfplay_peek", C.c_int, [C.c_void_p, C.POINTER(MzSelfPlayPeek)]),
+    ("mz_selfplay_set_opponent", C.c_int, [C.c_void_p, C.c_int32, C.c_int32]),
+    ("mz_debug_opponent_action", C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_void_p]),
     ("mz_debug_small_search_plan", C.c_int, [C.c_int32] * 10 + [C.POINTER(C.c_int64)]),
     ("mz_debug_conv3x3", C.c_int, [C.c_int, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p]),

@@ -14,8 +14,14 @@
 // [B][max_moves] and leave the device only when the game ends, as one packed block written by a warp straight into
 // mapped pinned host memory (no per-move D2H, no host-side bookkeeping per move).
 //
+// Evaluation games (mz_selfplay_set_opponent): MuZero plays muzero_player's side, a hard-coded opponent (the expert
+// scan of games/tictactoe.py:310-349 / games/connect4.py:307-348, or a uniformly random legal move) the other one.  Only
+// MuZero's moves are searched: the opponent replies inside the same step-kernel pass, so every slot reaches the next
+// batched search with MuZero to move.
+//
 // Random draws: Philox4x32-10 keyed by (seed, global game id, move): root noise and first-simulation ties inside the
-// search (tree.cuh), the action sample here (tag kTagAction), CartPole's reset state (tag kTagReset).
+// search (tree.cuh), the action sample here (tag kTagAction), CartPole's reset state (tag kTagReset), the opponent's
+// default move (tag kTagOpponent).
 #include <math.h>
 #include <stdio.h>
 #include <string.h>
@@ -26,10 +32,12 @@
 namespace mz {
 
 constexpr uint32_t kTagReset = 0x7169E004u;
+constexpr uint32_t kTagOpponent = 0x7169E005u;
 constexpr int kMaxCells = 48;              // board cells per slot (Connect4: 42)
 
 struct SpDev {
     int env, B, A, O, H, W, K, max_moves, threshold, reward_scale;
+    int opponent, muzero_player;           // MZ_OPPONENT_*; the side MuZero plays when the opponent is not "self"
     uint64_t seed;
     int64_t id_stride;         // a slot's next game id = current + id_stride
     int td_steps;              // > 0: PER priorities are computed while packing (replay_buffer.py:33-51)
@@ -251,16 +259,10 @@ MZ_DEVINL int sample_action(const SpDev& s, int g, double temperature, double u)
     return pick > last ? last : pick;                          // rounding can leave u >= cdf[-1]
 }
 
-// select_action + Game.step + record for slot g (one thread)
-MZ_DEVINL void slot_act(const SpDev& s, int g) {
+// Game.step + record of the slot's next move (one thread).  searched: the move was chosen by the search that just
+// finished (its root value and visit counts are recorded); otherwise it is an opponent's move: root value NaN, no visits
+MZ_DEVINL void slot_play(const SpDev& s, int g, int action, bool searched) {
     const int t = s.move[g];
-    const int64_t gid = s.game_id[g];
-    int action = s.forced_action ? s.forced_action[g] : -1;
-    if (action < 0) {
-        const double T = (s.threshold == 0 || t + 1 < s.threshold) ? s.temperature : 0.0;
-        const double u = s.uniform ? s.uniform[g] : philox_uniform53(s.seed, gid, t, 0u, kTagAction);
-        action = sample_action(s, g, T, u);
-    }
     float reward;
     bool done;
     if (s.env == MZ_ENV_CARTPOLE) {
@@ -273,8 +275,8 @@ MZ_DEVINL void slot_act(const SpDev& s, int g) {
     }
     // record of move t (store_search_statistics uses the pre-step root, self_play.py:169-175)
     const size_t r = (size_t)g * s.max_moves + t;
-    s.rec_root[r] = s.root_value[g];
-    for (int k = 0; k < s.A; ++k) s.rec_visits[r * s.A + k] = s.visits[(size_t)g * s.A + k];
+    s.rec_root[r] = searched ? s.root_value[g] : __longlong_as_double(0x7FF8000000000000ll);
+    for (int k = 0; k < s.A; ++k) s.rec_visits[r * s.A + k] = searched ? s.visits[(size_t)g * s.A + k] : 0;
     s.rec_action[r] = action;
     s.rec_reward[r] = reward;
     publish(s, g);
@@ -285,6 +287,107 @@ MZ_DEVINL void slot_act(const SpDev& s, int g) {
     s.move[g] = t + 1;
     s.last_action[g] = action;
     if (done || t + 1 >= s.max_moves) s.fin[g] = t + 1;
+}
+
+// select_action + Game.step + record for slot g (one thread)
+MZ_DEVINL void slot_act(const SpDev& s, int g) {
+    const int t = s.move[g];
+    const int64_t gid = s.game_id[g];
+    int action = s.forced_action ? s.forced_action[g] : -1;
+    if (action < 0) {
+        const double T = (s.threshold == 0 || t + 1 < s.threshold) ? s.temperature : 0.0;
+        const double u = s.uniform ? s.uniform[g] : philox_uniform53(s.seed, gid, t, 0u, kTagAction);
+        action = sample_action(s, g, T, u);
+    }
+    slot_play(s, g, action, true);
+}
+
+// ------------------------------------------------------------------------------------------
+// hard-coded opponents of evaluation games (SelfPlay.select_opponent_action, self_play.py:188-220), one warp per position
+// board: H*W stones (+1 / -1 / 0, row 0 = the bottom row), player: side to move (+1 / -1); every lane returns the move
+// ------------------------------------------------------------------------------------------
+// numpy.random.choice(legal_actions()) with the uniform u: floor(u * n_legal) over the legal actions in ascending order
+// (sample_action's T = inf rule); -1 when nothing is legal
+MZ_DEVINL int random_action(const int8_t* board, int env, double u, int lane) {
+    const bool c4 = env == MZ_ENV_CONNECT4;
+    const int A = c4 ? 7 : 9;
+    unsigned legal = __ballot_sync(0xffffffffu, lane < A && board[c4 ? 5 * 7 + lane : lane] == 0);
+    const int n = __popc(legal);
+    int idx = (int)(u * n);
+    if (idx >= n) idx = n - 1;
+    for (int i = 0; i < idx; ++i) legal &= legal - 1;
+    return __ffs(legal) - 1;
+}
+
+// The expert (games/_boards.py::_threat_scan with tictactoe.py / connect4.py::_expert_windows): the reference walks its
+// windows in order; a window whose stones sum to +-need has one gap, which becomes the candidate move if it is playable,
+// and is played at once if the window belongs to the side to move (a win); a later qualifying window overwrites the
+// candidate (a block); without one the random move is played.  Here lane L takes window 32c + L of chunk c: the first
+// chunk with a win plays its lowest such lane, otherwise the highest qualifying lane of the last chunk that has one.
+//   TicTacToe: 8 windows of 3 cells, need 2: row i then column i for i = 0..2, the diagonal, the anti-diagonal.
+//   Connect4: 120 windows of 4 cells, need 3: for every 4x4 sub-board (k = 0..2 rows up, l = 0..3 columns right) row i
+//   then column i for i = 0..3, the diagonal, the anti-diagonal.  A gap is playable only as the next free cell of its
+//   column; a vertical window names its column without looking at the gap.
+// The windows are index arithmetic rather than a table: a lookup per lane at 32 different addresses would serialise
+// on the constant cache.
+MZ_DEVINL int expert_action(const int8_t* board, int player, int env, double u, int lane) {
+    const bool c4 = env == MZ_ENV_CONNECT4;
+    const int H = c4 ? 6 : 3, W = c4 ? 7 : 3, len = c4 ? 4 : 3, need = c4 ? 3 : 2, n_windows = c4 ? 120 : 8;
+    int height = 0;                                   // Connect4: stones in column `lane` = row of its next free cell
+    if (c4 && lane < W)
+        for (int y = 0; y < H; ++y) height += board[y * W + lane] != 0;
+    int candidate = -1;
+    for (int base = 0; base < n_windows; base += 32) {
+        const int w = base + lane;
+        int y0, x0, dy = 0, dx = 0, fixed = -1;        // cells (y0 + j * dy, x0 + j * dx), j < len
+        if (c4) {
+            const int k = w / 40, l = (w / 10) % 4, r = w % 10, i = r >> 1;
+            if (r == 8) { y0 = k; x0 = l; dy = 1; dx = 1; }
+            else if (r == 9) { y0 = k; x0 = l + 3; dy = 1; dx = -1; }
+            else if (r & 1) { y0 = k; x0 = l + i; dy = 1; fixed = l + i; }
+            else { y0 = k + i; x0 = l; dx = 1; }
+        } else {
+            const int i = w >> 1;
+            if (w == 6) { y0 = 0; x0 = 0; dy = 1; dx = 1; }
+            else if (w == 7) { y0 = 0; x0 = 2; dy = 1; dx = -1; }
+            else if (w & 1) { y0 = 0; x0 = i; dy = 1; }
+            else { y0 = i; x0 = 0; dx = 1; }
+        }
+        int sum = 0, gy = 0, gx = 0;
+        if (w < n_windows)
+            for (int j = 0; j < len; ++j) {
+                const int y = y0 + j * dy, x = x0 + j * dx, v = board[y * W + x];
+                sum += v;
+                if (v == 0) { gy = y; gx = x; }
+            }
+        const int gap_height = c4 ? __shfl_sync(0xffffffffu, height, gx) : 0;
+        const bool qualifies = w < n_windows && (sum == need || sum == -need) && (!c4 || fixed >= 0 || gap_height == gy);
+        const int action = fixed >= 0 ? fixed : c4 ? gx : gy * W + gx;
+        const unsigned wins = __ballot_sync(0xffffffffu, qualifies && player * sum > 0);
+        if (wins) return __shfl_sync(0xffffffffu, action, __ffs(wins) - 1);
+        const unsigned blocks = __ballot_sync(0xffffffffu, qualifies);
+        if (blocks) candidate = __shfl_sync(0xffffffffu, action, 31 - __clz(blocks));
+    }
+    return candidate >= 0 ? candidate : random_action(board, env, u, lane);
+}
+
+MZ_DEVINL int opponent_action(const int8_t* board, int player, int env, int opponent, double u, int lane) {
+    return opponent == MZ_OPPONENT_EXPERT ? expert_action(board, player, env, u, lane) : random_action(board, env, u, lane);
+}
+
+// the opponent's move in slot g: the whole warp chooses it, lane 0 steps and records it; returns fin[g] after the move.
+// The caller has synchronised the warp after the slot's last write.
+MZ_DEVINL int opponent_move(const SpDev& s, int g, int lane) {
+    const double u = philox_uniform53(s.seed, s.game_id[g], s.move[g], 0u, kTagOpponent);
+    const int action = opponent_action(s.board + (size_t)g * kMaxCells, s.player[g], s.env, s.opponent, u, lane);
+    int T = 0;
+    if (lane == 0) {
+        slot_play(s, g, action, false);
+        T = s.fin[g];
+    }
+    T = __shfl_sync(0xffffffffu, T, 0);
+    __syncwarp();
+    return T;
 }
 
 __host__ __device__ inline unsigned long long staged_block_bytes(int T, int A, int O) {
@@ -328,10 +431,14 @@ MZ_DEVINL float initial_priority(const SpDev& s, int g, int T, int i) {
 // finishing warps per move: 89 us per launch at 4096 CartPole games, profiles/r02_selfplay_loop.md): the cursor may run
 // past the capacity, reservations that end beyond it are void (the game stays parked), and since the cursor only grows
 // the valid reservations are a contiguous prefix whose end is tracked in counters[5].
+// kOpponent (evaluation games): after MuZero's move the opponent replies in a game that goes on, and after a restart it
+// opens the next game when MuZero plays second, so the next search sees MuZero to move in every slot.  Self-play runs
+// the kOpponent = false instance, which has no opponent code.
 constexpr int kStepThreads = 1024;
 
+template <bool kOpponent>
 __global__ void __launch_bounds__(kStepThreads) selfplay_step_kernel(const SpDev s, int act) {
-    __shared__ int s_active;
+    __shared__ int s_active;                         // moves played by this CTA
     if (threadIdx.x == 0) s_active = 0;
     __syncthreads();
     const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -348,6 +455,10 @@ __global__ void __launch_bounds__(kStepThreads) selfplay_step_kernel(const SpDev
         }
         T = __shfl_sync(0xffffffffu, T, 0);
         __syncwarp();
+        if (kOpponent && act && T == 0) {            // MuZero moved and the game goes on (move + 1 < max_moves)
+            T = opponent_move(s, g, lane);
+            if (lane == 0) atomicAdd(&s_active, 1);
+        }
     }
     if (T != 0) {
         const unsigned long long bytes = staged_block_bytes(T, s.A, s.O);
@@ -404,10 +515,41 @@ __global__ void __launch_bounds__(kStepThreads) selfplay_step_kernel(const SpDev
             }
             __syncwarp();
             if (lane == 0) start_game(s, g, s.game_id[g] + s.id_stride);
+            if (kOpponent && s.muzero_player == 1) {  // the opponent plays move 0 of the slot's next game
+                __syncwarp();
+                opponent_move(s, g, lane);
+                if (lane == 0) atomicAdd(&s_active, 1);
+            }
         }
     }
     __syncthreads();
     if (threadIdx.x == 0 && s_active) atomicAdd(&s.counters[0], (unsigned long long)s_active);
+}
+
+static void launch_step(MzHandle* h, const SpDev& s, int act) {
+    const int blocks = (s.B * 32 + kStepThreads - 1) / kStepThreads;
+    if (s.opponent == MZ_OPPONENT_SELF) selfplay_step_kernel<false><<<blocks, kStepThreads, 0, h->stream>>>(s, act);
+    else selfplay_step_kernel<true><<<blocks, kStepThreads, 0, h->stream>>>(s, act);
+    h->launches += 1;
+}
+
+// move 0 of the games mz_selfplay_begin started, played by the opponent (one warp per slot)
+__global__ void selfplay_open_kernel(const SpDev s) {
+    const int g = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (g >= s.B) return;
+    opponent_move(s, g, lane);
+    if (lane == 0) atomicAdd(&s.counters[0], 1ull);
+}
+
+__global__ void opponent_debug_kernel(int env, int opponent, int n, const int8_t* board, const int8_t* player,
+                                      const double* uniform, int32_t* action) {
+    const int p = (blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+    const int lane = threadIdx.x & 31;
+    if (p >= n) return;
+    const int cells = env == MZ_ENV_CONNECT4 ? 42 : 9;
+    const int a = opponent_action(board + (size_t)p * cells, player[p], env, opponent, uniform[p], lane);
+    if (lane == 0) action[p] = a;
 }
 
 }  // namespace mz
@@ -426,6 +568,7 @@ struct MzSelfPlay {
     unsigned long long* d_index[2] = {nullptr, nullptr};
     int cur = 0;                               // area the next mz_selfplay_moves / enqueue writes
     bool in_flight = false;                    // moves enqueued, not waited for yet
+    bool moves_played = false;                 // moves enqueued or opening moves played since mz_selfplay_begin
     unsigned long long* h_counters = nullptr;  // pinned copy of the counters
     int32_t* d_forced = nullptr;
     double* d_uniform = nullptr;
@@ -598,17 +741,14 @@ static int sp_enqueue(MzHandle* h, int32_t n_moves, double temperature, const Mz
     call.add_noise = 1; call.noise = noise; call.first_index = first;
     call.game_id = s.game_id; call.move_index = s.move;
     call.visit_counts = s.visits; call.root_value = s.root_value;
+    sp->moves_played = true;
     MZ_CUDA(h, cudaEventRecord(sp->e0, h->stream));
-    if (sp->h_counters[4]) {                           // games parked by the previous call first, so their slots play again
-        selfplay_step_kernel<<<(B * 32 + kStepThreads - 1) / kStepThreads, kStepThreads, 0, h->stream>>>(s, 0);
-        h->launches += 1;
-    }
+    if (sp->h_counters[4]) launch_step(h, s, 0);      // games parked by the previous call first, so their slots play again
     MZ_CUDA(h, cudaMemsetAsync(s.counters + 4, 0, 8, h->stream));      // [4] = park events of THIS call
     for (int m = 0; m < n_moves; ++m) {
         int rc = mz_dispatch_search(h, call, false, false, 0);
         if (rc) return rc;
-        selfplay_step_kernel<<<(B * 32 + kStepThreads - 1) / kStepThreads, kStepThreads, 0, h->stream>>>(s, 1);
-        h->launches += 1;
+        launch_step(h, s, 1);
     }
     MZ_CUDA(h, cudaGetLastError());
     MZ_CUDA(h, cudaEventRecord(sp->e1, h->stream));
@@ -681,5 +821,60 @@ extern "C" int mz_selfplay_peek(MzHandle* h, const MzSelfPlayPeek* out) {
     if (out->game_id) MZ_CUDA(h, cudaMemcpy(out->game_id, s.game_id, B * 8, cudaMemcpyDeviceToHost));
     if (out->move_index) MZ_CUDA(h, cudaMemcpy(out->move_index, s.move, B * 4, cudaMemcpyDeviceToHost));
     if (out->last_action) MZ_CUDA(h, cudaMemcpy(out->last_action, s.last_action, B * 4, cudaMemcpyDeviceToHost));
+    return MZ_OK;
+}
+
+extern "C" int mz_selfplay_set_opponent(MzHandle* h, int32_t opponent, int32_t muzero_player) {
+    if (!h || !h->sp) return fail(h, MZ_ESTATE, "mz_selfplay_set_opponent: call mz_selfplay_begin first");
+    MzSelfPlay* sp = h->sp;
+    SpDev& s = sp->dev;
+    if (sp->moves_played) return fail(h, MZ_ESTATE, "mz_selfplay_set_opponent: moves already played, call mz_selfplay_begin first");
+    if (opponent != MZ_OPPONENT_SELF && opponent != MZ_OPPONENT_EXPERT && opponent != MZ_OPPONENT_RANDOM)
+        return fail(h, MZ_EINVAL, "mz_selfplay_set_opponent: unknown opponent");
+    if (muzero_player != 0 && muzero_player != 1) return fail(h, MZ_EINVAL, "mz_selfplay_set_opponent: muzero_player must be 0 or 1");
+    if (opponent != MZ_OPPONENT_SELF) {
+        if (s.env == MZ_ENV_CARTPOLE) return fail(h, MZ_EINVAL, "mz_selfplay_set_opponent: CartPole has one player, its opponent is \"self\"");
+        if (s.td_steps > 0)
+            return fail(h, MZ_EINVAL, "mz_selfplay_set_opponent: evaluation games are not for the replay buffer, td_steps must be 0");
+        if (s.max_moves < 2) return fail(h, MZ_EINVAL, "mz_selfplay_set_opponent: max_moves < 2 leaves no move to MuZero");
+    }
+    MZ_CUDA(h, cudaSetDevice(h->device));
+    s.opponent = opponent;
+    s.muzero_player = opponent == MZ_OPPONENT_SELF ? 0 : muzero_player;
+    if (s.opponent != MZ_OPPONENT_SELF && s.muzero_player == 1) {
+        selfplay_open_kernel<<<(s.B * 32 + 255) / 256, 256, 0, h->stream>>>(s);
+        h->launches += 1;
+        MZ_CUDA(h, cudaGetLastError());
+        MZ_CUDA(h, cudaStreamSynchronize(h->stream));
+        sp->moves_played = true;
+    }
+    return MZ_OK;
+}
+
+extern "C" int mz_debug_opponent_action(int device, int32_t env, int32_t opponent, int32_t n, const int8_t* board,
+                                        const int8_t* player, const double* uniform, int32_t* action) {
+    if (!board || !player || !uniform || !action || n < 0) return fail(nullptr, MZ_EINVAL, "mz_debug_opponent_action: bad argument");
+    if (env != MZ_ENV_TICTACTOE && env != MZ_ENV_CONNECT4)
+        return fail(nullptr, MZ_EINVAL, "mz_debug_opponent_action: env must be MZ_ENV_TICTACTOE or MZ_ENV_CONNECT4");
+    if (opponent != MZ_OPPONENT_EXPERT && opponent != MZ_OPPONENT_RANDOM)
+        return fail(nullptr, MZ_EINVAL, "mz_debug_opponent_action: opponent must be MZ_OPPONENT_EXPERT or MZ_OPPONENT_RANDOM");
+    if (n == 0) return MZ_OK;
+    if (cudaSetDevice(device) != cudaSuccess) return fail(nullptr, MZ_ECUDA, "mz_debug_opponent_action: no such device");
+    const size_t cells = env == MZ_ENV_CONNECT4 ? 42 : 9;
+    const size_t o_player = (size_t)n * cells, o_uniform = (o_player + n + 7) & ~(size_t)7, o_action = o_uniform + 8 * (size_t)n;
+    unsigned char* d = nullptr;
+    if (cudaMalloc(&d, o_action + 4 * (size_t)n) != cudaSuccess) return fail(nullptr, MZ_ENOMEM, "mz_debug_opponent_action: out of device memory");
+    cudaError_t e = cudaMemcpy(d, board, o_player, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(d + o_player, player, n, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) e = cudaMemcpy(d + o_uniform, uniform, 8 * (size_t)n, cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        opponent_debug_kernel<<<(int)(((size_t)n * 32 + 255) / 256), 256>>>(
+            env, opponent, n, reinterpret_cast<const int8_t*>(d), reinterpret_cast<const int8_t*>(d + o_player),
+            reinterpret_cast<const double*>(d + o_uniform), reinterpret_cast<int32_t*>(d + o_action));
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess) e = cudaMemcpy(action, d + o_action, 4 * (size_t)n, cudaMemcpyDeviceToHost);
+    cudaFree(d);
+    if (e != cudaSuccess) return fail(nullptr, MZ_ECUDA, std::string("mz_debug_opponent_action: ") + cudaGetErrorString(e));
     return MZ_OK;
 }

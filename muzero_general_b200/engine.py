@@ -362,12 +362,17 @@ class DeviceSelfPlayLoop:
     finished games handed back as packed struct-of-arrays blocks (SURVEY.md 8f-1, include/mzb200.h)."""
 
     ENVS = {"cartpole": _lib.MZ_ENV_CARTPOLE, "tictactoe": _lib.MZ_ENV_TICTACTOE, "connect4": _lib.MZ_ENV_CONNECT4}
+    OPPONENTS = {"self": _lib.MZ_OPPONENT_SELF, "expert": _lib.MZ_OPPONENT_EXPERT, "random": _lib.MZ_OPPONENT_RANDOM}
 
     def __init__(self, engine: SearchEngine, env: str, max_moves: int, temperature_threshold=None, reward_scale: int = 1,
                  first_game_id: int = 0, staging_bytes: int = 0, game_id_stride: int = 0, td_steps: int = 0,
-                 per_alpha: float = 1.0, discount: float = 1.0):
+                 per_alpha: float = 1.0, discount: float = 1.0, opponent: str = "self", muzero_player: int = 0):
+        """``opponent`` = "expert" / "random" plays evaluation games (``mz_selfplay_set_opponent``): MuZero searches the
+        moves of side ``muzero_player`` only, the hard-coded opponent plays the other side on the device."""
         if env not in self.ENVS:
             raise NotImplementedError(f"no device-resident environment for {env!r}")
+        if opponent not in self.OPPONENTS:
+            raise ValueError(f"opponent must be one of {sorted(self.OPPONENTS)}, got {opponent!r}")
         self.engine = engine
         d = _lib.MzSelfPlayDesc()
         d.env = self.ENVS[env]
@@ -384,6 +389,9 @@ class DeviceSelfPlayLoop:
         self.with_priorities = bool(d.td_steps)
         d.staging_bytes = int(staging_bytes)
         engine._check(engine.lib.mz_selfplay_begin(engine._h, C.byref(d)))
+        if opponent != "self":
+            engine._check(engine.lib.mz_selfplay_set_opponent(engine._h, self.OPPONENTS[opponent], int(muzero_player)))
+        self.opponent, self.muzero_player = opponent, int(muzero_player)
         self.stats = _lib.MzSelfPlayStats()
 
     def moves(self, n_moves: int, temperature: float, forced_action=None, uniform=None, noise=None, first_index=None):
@@ -469,6 +477,23 @@ def parse_staged_games(buf: bytes, index):
     for g, meta in zip(games, index[:, 1]):
         assert (int(meta) >> 32, int(meta) & 0xFFFFFFFF) == (g["slot"], g["length"])
     return games
+
+
+def debug_opponent_action(env, opponent, board, player, uniform, device=0):
+    """The device's hard-coded opponent (``mz_debug_opponent_action``, the function the evaluation loop plays with) on n
+    positions: ``env`` "tictactoe" / "connect4", ``opponent`` "expert" / "random", ``board`` [n, H*W] (+1 / -1 / 0, row 0
+    at the bottom), ``player`` [n] side to move (+1 / -1), ``uniform`` [n] the default move's draw.  Returns int32 [n]."""
+    lib = _lib.load_library()
+    board = numpy.ascontiguousarray(board, numpy.int8)
+    n = board.shape[0]
+    player = numpy.ascontiguousarray(player, numpy.int8).reshape(n)
+    uniform = numpy.ascontiguousarray(uniform, numpy.float64).reshape(n)
+    out = numpy.empty(n, numpy.int32)
+    rc = lib.mz_debug_opponent_action(device, DeviceSelfPlayLoop.ENVS[env], DeviceSelfPlayLoop.OPPONENTS[opponent], n,
+                                      board.ctypes.data, player.ctypes.data, uniform.ctypes.data, out.ctypes.data)
+    if rc != 0:
+        raise _lib.MzError(rc, lib.mz_last_error(None).decode())
+    return out
 
 
 def debug_conv3x3(x, w, bias=None, residual=None, relu=False, tensor_cores=False, device=0):

@@ -10,6 +10,10 @@ side so stock reference configs load unchanged:
 * ``num_parallel_games``  games searched in lockstep per GPU process (default 1)
 * ``rng_mode``            "numpy" (reference draw order on legacy per-game streams) or
                           "philox" (counter-based, generated on the device)
+* ``test_games_per_report``  evaluation games the test worker plays per weight refresh
+                          (``SelfPlay.play_test_games``); absent or 0 = one ``play_game`` as in the reference
+* ``test_parallel_games`` slots of the device engine that plays evaluation games (default 4096,
+                          never more than the games asked for)
 """
 import datetime
 import pathlib

@@ -373,8 +373,16 @@ class PackedGameHistory(GameHistory):
         d["reward_history"] = [0] + [reward_type(r) for r in g["reward"].tolist()]
         d["to_play_history"] = [int(g["first_to_play"])] + g["to_play"].tolist()
         visits = g["visits"]
-        d["child_visits"] = (visits / visits.sum(1, keepdims=True)).tolist()
-        d["root_values"] = g["root_value"].tolist()
+        searched = visits.sum(1) > 0
+        if searched.all():
+            d["child_visits"] = (visits / visits.sum(1, keepdims=True)).tolist()
+            d["root_values"] = g["root_value"].tolist()
+        else:
+            # evaluation games: the opponent's moves carry no search statistics, like store_search_statistics(None, ...)
+            # (self_play.py:175,496-511): no child_visits row, root value None
+            visits = visits[searched]
+            d["child_visits"] = (visits / visits.sum(1, keepdims=True)).tolist()
+            d["root_values"] = [v if ok else None for v, ok in zip(g["root_value"].tolist(), searched.tolist())]
 
     def __reduce__(self):
         self._materialise()
@@ -404,6 +412,7 @@ class SelfPlay:
 
     def __init__(self, initial_checkpoint, Game, config, seed, device=0, first_game_id=0, game_id_stride=None):
         self.config = config
+        self.device = device
         self.first_game_id = int(first_game_id)      # rank * num_parallel_games in a multi-GPU job
         # a slot's next game takes (current id + stride): world_size * num_parallel_games keeps ids unique over ranks
         self.game_id_stride = int(game_id_stride or getattr(config, "num_parallel_games", 1) or 1)
@@ -423,6 +432,9 @@ class SelfPlay:
         self._stream = None           # across play_games calls (its generator)
         self.played_games = 0
         self.played_steps = 0
+        self._test_model = None       # evaluation games on the device (play_test_games): own engine, own game ids
+        self._next_test_game_id = 0
+        self.last_test_searches = 0   # positions the last device evaluation searched, games dropped beyond the ids included
 
     # ------------------------------------------------------------------ reference loop
     def continuous_self_play(self, shared_storage, replay_buffer, test_mode=False):
@@ -445,6 +457,12 @@ class SelfPlay:
                 else:
                     game_history = self.play_game(temperature, cfg.temperature_threshold, False, "self", 0)
                     _fire(replay_buffer, "save_game", game_history, shared_storage)
+            elif int(getattr(cfg, "test_games_per_report", 0) or 0):
+                # a batch of evaluation games per weight refresh: the reference's keys averaged over the games
+                _, summary = self.play_test_games(int(cfg.test_games_per_report))
+                _fire(shared_storage, "set_info", {k: summary[k] for k in ("episode_length", "total_reward", "mean_value")})
+                if 1 < len(cfg.players):
+                    _fire(shared_storage, "set_info", {k: summary[k] for k in ("muzero_reward", "opponent_reward")})
             else:
                 # Take the best action (no exploration) in test mode
                 game_history = self.play_game(
@@ -549,6 +567,62 @@ class SelfPlay:
         raise NotImplementedError(
             'Wrong argument: "opponent" argument should be "self", "human", "expert" or "random"')
 
+    # ------------------------------------------------------------------ evaluation games
+    def play_test_games(self, num_games, opponent=None, muzero_player=None, first_game_id=None):
+        """``num_games`` evaluation games, the batched ``MuZero.test`` (muzero.py:369-424) and test worker
+        (self_play.py:54-90): greedy moves with root noise, as ``play_game(0, 0, False, opponent, muzero_player)``.
+
+        ``opponent`` / ``muzero_player`` = None take ``config.opponent`` / ``config.muzero_player`` (an explicit 0 is
+        kept); one-player games always play "self"; "human" is not supported.  Returns ``(games, summary)``: the games
+        (``PackedGames`` from the device loop, else a list of ``GameHistory``) and ``evaluation_summary`` of them.
+
+        With a device-resident environment (``loop_path == "device"``) the games run in ``mz_selfplay_*`` on an engine of
+        their own with ``min(num_games, config.test_parallel_games or 4096)`` slots, loaded with the worker's current
+        weights; the self-play batch in flight is not touched.  Exactly the global game ids ``[first_game_id,
+        first_game_id + num_games)`` are returned (games the slots start beyond them are dropped), so the result does not
+        depend on the number of slots; ``first_game_id`` = None continues after the previous call.  Otherwise
+        ``play_game`` is called ``num_games`` times."""
+        cfg = self.config
+        opponent, muzero_player = resolve_opponent(cfg, opponent, muzero_player)
+        num_games = int(num_games)
+        first = self._next_test_game_id if first_game_id is None else int(first_game_id)
+        if self._device_env_name():
+            games = self._device_test_games(num_games, opponent, muzero_player, first)
+        else:
+            games = [self.play_game(0, 0, False, opponent, muzero_player) for _ in range(num_games)]
+        self._next_test_game_id = first + num_games
+        return games, evaluation_summary(games, len(cfg.players), muzero_player)
+
+    def _device_test_games(self, num_games, opponent, muzero_player, first):
+        cfg, Game = self.config, self.Game
+        B = max(1, min(num_games, int(getattr(cfg, "test_parallel_games", 0) or 4096)))
+        if self._test_model is None or self._test_model.engine.max_games != B:
+            if self._test_model is not None:
+                self._test_model.engine.close()
+            self._test_model = DeviceModel(cfg, max_games=B, device=self.device, seed=self.seed)
+        self._test_model.set_weights(self.model.get_weights())
+        vec = getattr(Game, "VECTOR", None)
+        loop = DeviceSelfPlayLoop(self._test_model.engine, Game.DEVICE_ENV, cfg.max_moves,
+                                  reward_scale=getattr(vec, "REWARD_SCALE", 1), first_game_id=first, game_id_stride=B,
+                                  opponent=opponent, muzero_player=muzero_player)
+        out = PackedGames(tuple(cfg.observation_shape), getattr(vec, "OBS_DTYPE", numpy.float32),
+                          int if vec is not None else float)
+        end = first + num_games
+        searches = 0
+        while len(out) < num_games:
+            # one batched move per call: the evaluation stops right after the last wanted game ends (a move costs a
+            # search of the whole batch, the host round trip is small beside it)
+            loop.moves(1, 0.0)
+            searches += 1
+            buf, index = loop.drain()
+            if len(index):
+                ids = numpy.frombuffer(buf, numpy.int64)[(index[:, 0] // 8).astype(numpy.int64)]
+                out.add(buf, index[ids < end])
+        self.played_games += len(out)
+        self.played_steps += out.total_moves
+        self.last_test_searches = searches * B
+        return out
+
     @staticmethod
     def select_action(node, temperature):
         """Visit-count sampling (self_play.py:222-245)."""
@@ -633,6 +707,62 @@ class SelfPlay:
 
     def close(self):
         self.model.engine.close()
+
+
+def resolve_opponent(config, opponent=None, muzero_player=None):
+    """(opponent, muzero_player) of an evaluation: None takes the config's value (an explicit 0 is kept, where
+    muzero.py:390's ``if muzero_player`` would replace it); a one-player game plays "self" (self_play.py:60)."""
+    if opponent == "human":
+        raise ValueError('opponent "human" is interactive: use play_game for it')
+    opponent = config.opponent if opponent is None else opponent
+    muzero_player = int(config.muzero_player if muzero_player is None else muzero_player)
+    if len(config.players) == 1:
+        return "self", muzero_player
+    if opponent not in ("self", "expert", "random"):
+        raise ValueError(f'opponent must be "self", "expert" or "random", got {opponent!r}')
+    return opponent, muzero_player
+
+
+def evaluation_summary(games, num_players, muzero_player):
+    """Test-worker statistics (self_play.py:67-90) of every game, averaged over the games, plus ``MuZero.test``'s
+    ``result`` (muzero.py:411-424).  ``games``: ``GameHistory`` objects or ``PackedGames`` (read from the packed reward /
+    to_play / root-value arrays, nothing materialised).  Per game, as the reference computes it:
+      episode_length = moves; total_reward = sum of rewards; mean_value = mean of the root values that are truthy
+      (neither None nor 0.0; NaN for a game without one); muzero_reward / opponent_reward = rewards of the moves played by
+      muzero_player / the other side.
+    A game whose mean_value is NaN is left out of that average.  Two-player games also get the keys muzero_reward,
+    opponent_reward and wins / draws / losses (muzero_reward above / equal to / below opponent_reward)."""
+    rows = []                 # per game: length, total reward, mean value, muzero reward, opponent reward
+    if isinstance(games, PackedGames):
+        for g in games.blocks():
+            rewards = g["reward"].astype(numpy.float64)
+            mover = numpy.concatenate(([g["first_to_play"]], g["to_play"][:-1]))
+            root = g["root_value"]
+            values = root[~numpy.isnan(root) & (root != 0)]
+            rows.append((g["length"], float(rewards.sum()), float(values.mean()) if values.size else numpy.nan,
+                         float(rewards[mover == muzero_player].sum()), float(rewards[mover != muzero_player].sum())))
+    else:
+        for h in games:
+            rh, tp = h.reward_history, h.to_play_history
+            values = [value for value in h.root_values if value]
+            with numpy.errstate(invalid="ignore", divide="ignore"):
+                mean_value = float(numpy.mean(values)) if values else numpy.nan
+            rows.append((len(h.action_history) - 1, sum(rh), mean_value,
+                         sum(reward for i, reward in enumerate(rh) if tp[i - 1] == muzero_player),
+                         sum(reward for i, reward in enumerate(rh) if tp[i - 1] != muzero_player)))
+    n = len(rows)
+    col = (lambda k: numpy.array([r[k] for r in rows], numpy.float64)) if n else (lambda k: numpy.zeros(0))
+    mean = lambda a: float(numpy.mean(a)) if a.size else numpy.nan
+    mv = col(2)
+    mv = mv[~numpy.isnan(mv)]
+    out = dict(num_games=n, episode_length=mean(col(0)), total_reward=mean(col(1)), mean_value=mean(mv))
+    if num_players > 1:
+        mine, theirs = col(3), col(4)
+        out.update(muzero_reward=mean(mine), opponent_reward=mean(theirs), wins=int((mine > theirs).sum()),
+                   draws=int((mine == theirs).sum()), losses=int((mine < theirs).sum()), result=mean(mine))
+    else:
+        out["result"] = out["total_reward"]
+    return out
 
 
 def _sample_action(actions, visit_counts, temperature, rng):
@@ -788,6 +918,12 @@ class PackedGames:
 
     def _make(self, buf, off):
         return PackedGameHistory(parse_staged_game(buf, int(off)), *self._args)
+
+    def blocks(self):
+        """The games as ``parse_staged_game`` dicts (numpy views of the packed arrays), no history objects."""
+        for buf, index in self._chunks:
+            for off in index[:, 0]:
+                yield parse_staged_game(buf, int(off))
 
     def __iter__(self):
         for buf, index in self._chunks:
