@@ -130,7 +130,13 @@ __global__ void __launch_bounds__(kFcMaxThreads) fc_search_kernel(const __grid_c
         // ------------------------------------------------------------------ simulations
         int max_depth = 0;
         for (int sim = 0; sim < N; ++sim) {
-            const Leaf leaf = tree_select<G>(c, t, sim, game_id, move, first_index);
+            Leaf leaf;
+            if constexpr (lookahead_levels<G>() >= 2) {
+                if (a.lookahead) leaf = tree_select_lookahead<G>(c, t, sim, game_id, move, first_index);
+                else leaf = tree_select<G>(c, t, sim, game_id, move, first_index);
+            } else {
+                leaf = tree_select<G>(c, t, sim, game_id, move, first_index);
+            }
             float value, reward;
             if (kTeacher) {
                 value = a.teacher.value[(size_t)g * N + sim];
@@ -250,8 +256,11 @@ static cudaError_t launch_one(const FcSearchArgs& a, int sm_count, size_t smem_c
 // shapes with a fully unrolled network path: games/cartpole.py (encoding 8, hidden 16, support 10, 2 actions)
 using CartPoleShape = FcFixedShape<8, 16, 10, 2>;
 
-cudaError_t launch_fc_search(const FcSearchArgs& a, int group, bool teacher, int sm_count, size_t smem_cap,
+cudaError_t launch_fc_search(const FcSearchArgs& args, int group, bool teacher, int sm_count, size_t smem_cap,
                              cudaStream_t stream, FcLaunchInfo* info) {
+    FcSearchArgs a = args;
+    const char* la = getenv("MZ_FC_LOOKAHEAD");                // A/B switch: 0 selects one tree level per round
+    a.lookahead = (a.A <= 2 && !(la && la[0] == '0')) ? 1 : 0;
     const char* generic = getenv("MZ_FC_GENERIC");             // A/B switch: always walk the layer descriptors
     if (!teacher && !(generic && generic[0] == '1') && fc_matches_fixed<CartPoleShape>(a.net)) {
         if (group == 16) return launch_one<16, false, CartPoleShape>(a, sm_count, smem_cap, stream, info);

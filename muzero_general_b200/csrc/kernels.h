@@ -80,6 +80,7 @@ struct FcSearchArgs {
     DevTeacher teacher;
     DevTrace trace;
     NodePool pool;         // pool.visit == nullptr unless MZ_FLAG_KEEP_TREE
+    int lookahead;         // set by launch_fc_search: several tree levels per selection round (|A| <= 2, tree.cuh)
 };
 
 struct FcInferArgs {

@@ -247,6 +247,128 @@ MZ_DEVINL Leaf tree_select(const TreeConst& c, GameTree& t, int sim, int64_t gam
 }
 
 // ------------------------------------------------------------------------------------------
+// Lookahead selection for |A| <= 2 (shared-memory trees): the same descent as tree_select, K levels per round.
+// With sibling width W = 2 only 2 lanes of the group score a level; here level l of a round (l = 0..K-1) is scored by
+// the 2^(l+1) lanes starting at lane 2^(l+1) - 2, one lane per grandchild path: lane local index j = 2*p + a scores child
+// a of the node reached by the action bits of p (most significant = level 0).  K = 2 (G = 8), 3 (G = 16: lanes 0-1,
+// 2-5, 6-13) or 4 (G = 32).  Every lane reaches its node by chasing at most K-1 expansion ids from the round's start
+// and gives up (score -inf) below an unexpanded one.  Each score is the one tree_select would compute at that node
+// (same loads, same operations, same order; the tree does not change during selection), so one xor-butterfly and one
+// ballot serve all levels, and the path is resolved level by level as uniform integer work on the ballot: tie count,
+// Philox tie draw with the true depth, tie counter on the resolved path only, and stop at the first unexpanded pick.
+// The next round starts from the last pick.  Bit-identical to tree_select<G, false>; only unread scores are added.
+// ------------------------------------------------------------------------------------------
+template <int G>
+constexpr int lookahead_levels() { return G >= 32 ? 4 : G >= 16 ? 3 : G >= 8 ? 2 : 1; }
+
+template <int G>
+MZ_DEVINL Leaf tree_select_lookahead(const TreeConst& c, GameTree& t, int sim, int64_t game_id, int move, int first_index) {
+    constexpr int K = lookahead_levels<G>();
+    static_assert(K >= 2, "lookahead needs at least two levels per round");
+    const int k = LaneGroup<G>::lane();
+    const int A = c.A;                                  // 1 or 2
+    int e = 0;
+    int n_parent = t.root_visit;
+    int depth = 0;
+    Leaf leaf;
+    if (k == 0) { t.path[0] = -1; t.path_reward[0] = t.root_reward; }
+    while (true) {
+        // this lane's level l and local index j inside it: lanes [2^(l+1) - 2, 2^(l+2) - 2); unused lanes get l = K.
+        // Recomputed every round from an opaque copy of the lane id: hoisted out of the simulation loop they would stay
+        // live through the network evaluation, where the fixed-shape kernel has no register to spare.
+        int kr = k;
+        asm volatile("" : "+r"(kr));
+        const int j = kr + 2 - (2 << (30 - __clz(kr + 2)));
+        const int lvl = (kr < (2 << K) - 2 && (A == 2 || j == 0)) ? 30 - __clz(kr + 2) : K;   // |A| = 1: only action 0
+        // 1. reach this lane's node (-1 if an ancestor is unexpanded): the ancestors' actions are the higher bits of j
+        int node = lvl < K ? e : -1, np = n_parent;
+#pragma unroll
+        for (int i = 0; i < K - 1; ++i) {
+            if (i < lvl && node >= 0) {
+                const int s = node * A + ((j >> (lvl - i)) & 1);
+                np = t.visit[s];
+                node = t.expansion[s];
+            }
+        }
+        // 2.-3. this lane's child: tree_select's score
+        const int a_own = j & 1;
+        const int slot_k = node * A + a_own;
+        const bool root_level = (node == 0);            // only the round's level 0 can sit at the root
+        const bool valid = node >= 0 && (!root_level || ((t.legal >> a_own) & 1u));
+        double score = -INFINITY;
+        int nc = 0, child_exp_k = -1;
+        float reward_k = 0.0f;
+        if (valid) {
+            nc = t.visit[slot_k];
+            child_exp_k = t.expansion[slot_k];
+            const double pr = root_level ? t.root_prior[a_own] : (double)t.prior[slot_k];
+            double pbc;
+            if (c.ucb) {
+                pbc = __ldg(c.ucb + np * (c.N + 2) + nc);
+            } else {
+                const double q = __ddiv_rn(c.sqrtn[np], (double)(nc + 1));
+                pbc = __dmul_rn(c.pbc[np], q);
+            }
+            score = __dmul_rn(pbc, pr);
+            if (nc > 0) {
+                reward_k = t.reward[slot_k];
+                const double v = value_range_normalize(t.mval[slot_k], t.lo, t.hi);
+                score = __dadd_rn(score, v);
+            } else {
+                score = __dadd_rn(score, 0.0);
+            }
+        }
+        // 4. sibling max of every level at once (siblings are lanes 2i, 2i+1), then one ballot for all levels
+        const double best = fmax(score, shfl_xor_f64(LaneGroup<G>::mask(), score, 1, G));
+        const unsigned tied = LaneGroup<G>::ballot(valid && score == best);
+        const unsigned expanded = LaneGroup<G>::ballot(child_exp_k >= 0);
+        // 5. resolve the path (uniform); the lane that scored a picked child writes its path entry
+        int pl = 0;
+        int p = 0;                                       // local index of the path node inside the next level
+#pragma unroll
+        for (int l = 0; l < K; ++l) {
+            const int pair = (2 << l) - 2 + 2 * p;       // first lane of the sibling pair below the path node
+            const unsigned tl = (tied >> pair) & 3u;
+            const int n_tied = __popc(tl);
+            int pick;
+            if (n_tied <= 1) {
+                pick = max(__ffs(tl) - 1, 0);
+            } else {
+                int idx;
+                const int d = depth + l;
+                if (sim == 0 && d == 0 && first_index >= 0) {
+                    idx = first_index < n_tied ? first_index : n_tied - 1;
+                } else {
+                    idx = philox_tie_index(c.seed, game_id, move, sim, d, n_tied);
+                    if (!(sim == 0 && d == 0)) t.ties += 1;
+                }
+                pick = nth_set_bit(tl, idx);
+            }
+            pl = pair + pick;
+            if (k == pl) { t.path[depth + l + 1] = slot_k; t.path_reward[depth + l + 1] = reward_k; }
+            if (!((expanded >> pl) & 1u)) break;
+            p = 2 * p + pick;
+        }
+        // 6. continue below the last pick, or stop at it
+        const int child_exp = LaneGroup<G>::bcast(child_exp_k, pl);
+        const int child_visits = LaneGroup<G>::bcast(nc, pl);
+        const int slot = LaneGroup<G>::bcast(slot_k, pl);
+        depth += 31 - __clz(pl + 2);                     // levels resolved in this round: level of lane pl, plus one
+        if (child_exp < 0) {
+            leaf.depth = depth;
+            leaf.parent_exp = (A == 2) ? (slot >> 1) : slot;
+            leaf.action = (A == 2) ? (slot & 1) : 0;
+            leaf.slot = slot;
+            break;
+        }
+        n_parent = child_visits;
+        e = child_exp;
+    }
+    LaneGroup<G>::sync();
+    return leaf;
+}
+
+// ------------------------------------------------------------------------------------------
 // Expansion of the selected leaf with the network outputs (self_play.py:345-351, 451-465).
 // prior_f32: this lane's fp32 softmax prior (lane k <-> action k).
 // ------------------------------------------------------------------------------------------
